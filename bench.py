@@ -1,6 +1,6 @@
 """Benchmark of the Stable Audio denoising hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config {2,3,4,5}] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config {2,3,4,5}] [--impl reference] [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[2] (--config 3, the configuration the metric is quoted on): Stable Audio
 Open 1.0 DiT (1.06 B parameters, random init), 47.55 s stereo 44.1 kHz = 1024 latent tokens, batch 4 per GPU with
@@ -219,6 +219,25 @@ def build_models(device):
     return wrapper, dec
 
 
+DUMP_MAX_ELEMENTS = 1 << 22        # per array: 16 MB of float32, so the three dumped arrays stay under 64 MB
+
+
+def dump_outputs(directory, outputs):
+    """Write each output as <directory>/<name>.npy in float32.  An array larger than DUMP_MAX_ELEMENTS is written as a
+    fixed seeded sample of its flattened elements (the same positions in every run of the same configuration), so
+    that the dumps of two builds can be compared element for element."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in outputs.items():
+        flat = t.detach().reshape(-1)
+        if flat.numel() > DUMP_MAX_ELEMENTS:
+            idx = torch.randint(flat.numel(), (DUMP_MAX_ELEMENTS,), generator=torch.Generator().manual_seed(0))
+            flat = flat[idx.sort().values.to(flat.device)]
+        else:
+            flat = flat.reshape(t.shape)
+        np.save(os.path.join(directory, name + ".npy"), flat.float().cpu().numpy())
+
+
 def cpu_baseline_leg():
     """Same bounded sample as --impl reference, ~10-20 s of host time."""
     do, cfg, sd, (x, t, c, ge), d, threads = cpu_sample(6.0, 1)
@@ -329,6 +348,7 @@ def run_native(args):
     barrier()
     wall1 = time.time()
     launches = _native.launch_count() - launches0
+    outputs = {"latents": loop.x, "denoised": loop.st.den_1}     # what the last timed step returned / estimated
     elapsed_ms = e0.elapsed_time(e1)
     clocks = sampler.stop(wall0, wall1) if rank == 0 else None
     if dist:
@@ -404,6 +424,7 @@ def run_native(args):
             audio = dec(lat[b:b + 1])
     d1.record()
     torch.cuda.synchronize()
+    outputs["decoded_audio"] = audio
     decode_ms = d0.elapsed_time(d1) / 3
     if dist:
         tmax = torch.tensor([decode_ms], device=device)
@@ -462,6 +483,8 @@ def run_native(args):
         if dist:
             td.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
 
     # ---------------- roofline of the dominant kernel (FF-in GEMM, tensor bound) --------------
     peaks = {}
@@ -564,9 +587,17 @@ def main():
     ap.add_argument("--no-cpu-baseline", dest="no_cpu_baseline", action="store_true")
     ap.add_argument("--no-graph", dest="no_graph", action="store_true", help="enqueue every kernel of a step instead of "
                     "replaying the captured CUDA graph of the denoiser call")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps write, as DIR/<name>.npy (float32), rank 0's latents and denoised "
+                         "estimate of the last timed step and its last decoded clip; inputs are seeded, so the same "
+                         "arguments give the same inputs in every run")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     set_config(args.config)
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the native path only")
         run_reference(args)
     else:
         if int(os.environ.get("WORLD_SIZE", "1")) > 1:

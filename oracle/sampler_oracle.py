@@ -158,8 +158,8 @@ def sample_dpmpp_3m_sde(model, x, sigmas, extra_args=None, callback=None, disabl
 
 
 # ---------------------------------------------------------------------------------------------
-# The reference's own sampler front end and inpainting mask (these ARE under /root/reference and are pinned
-# against the live reference by tests/test_oracle_vs_reference.py).
+# The reference's own sampler front end and inpainting mask (these ARE part of the reference and are pinned
+# against its outputs by tests/test_oracle_vs_reference.py).
 # ---------------------------------------------------------------------------------------------
 def get_bmask(i, steps, mask):
     """inference/sampling.py:120-124: hard mask that shrinks as the step index grows."""

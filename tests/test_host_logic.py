@@ -8,7 +8,7 @@ import sys
 import pytest
 import torch
 
-from helpers import rel_l2
+from helpers import load_golden, rel_l2
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -99,43 +99,25 @@ def test_get_conditioning_inputs_routing():
                         "negative_input_concat_cond"}
 
 
-class _FakeEnc(torch.nn.Module):
-    """average-pool 'encoder' (ratio 4, 2 -> 3 channels) so the chunking logic runs on CPU"""
-
-    def forward(self, x):
-        p = torch.nn.functional.avg_pool1d(x, 4)
-        return torch.cat([p, p[:, :1] * 0.5 - 3.0], dim=1)
-
-
-class _FakeDec(torch.nn.Module):
-    def forward(self, z):
-        return torch.repeat_interleave(z[:, :2] + z[:, 2:3] * 0.25, 4, dim=-1)
-
-
 def test_chunked_encode_decode_reconstruct_match_reference_or_closed_form():
     """With linear, position-wise fake encoder/decoder the Bartlett cross-fade weights sum to one on
-    the overlaps, so chunked == unchunked away from the padded tail; when /root/reference is present
-    the reference AudioAutoencoder is driven with the same fakes and must agree bit-for-bit."""
-    from oracle import ref_shims
+    the overlaps, so chunked == unchunked away from the padded tail; the reference AudioAutoencoder driven
+    with the same fakes (tests/golden/chunked_fake_autoencoder.npz) gave the same tensors bit for bit."""
+    from oracle.make_golden import FakeDecoder, FakeEncoder
     from stable_audio_tools.models.autoencoders import AudioAutoencoder
-    ae = AudioAutoencoder(_FakeEnc(), _FakeDec(), latent_dim=3, downsampling_ratio=4, sample_rate=16000, io_channels=2,
-                          bottleneck=None)
-    torch.manual_seed(0)
-    a = torch.randn(2, 2, 4 * 37)
-    z = torch.randn(2, 3, 41)
+    ae = AudioAutoencoder(FakeEncoder(), FakeDecoder(), latent_dim=3, downsampling_ratio=4, sample_rate=16000,
+                          io_channels=2, bottleneck=None)
+    g = load_golden("chunked_fake_autoencoder.npz")
+    a, z = torch.from_numpy(g["a"]), torch.from_numpy(g["z"])
     enc_c = ae.encode_audio(a.clone(), chunked=True, chunk_size=8, overlap=2, max_batch_size=3)
     dec_c = ae.decode_audio(z.clone(), chunked=True, chunk_size=8, overlap=2, max_batch_size=2)
     rec_c = ae.reconstruct_audio(a.clone(), chunked=True, chunk_size=8, overlap=2, max_batch_size=4)
     assert enc_c.shape == (2, 3, 37) and dec_c.shape == (2, 2, 41 * 4) and rec_c.shape == a.shape
     assert rel_l2(enc_c, ae.encode_audio(a, chunked=False)) < 1e-5
     assert rel_l2(dec_c, ae.decode_audio(z, chunked=False)) < 1e-5
-    if ref_shims.reference_available():
-        ref = ref_shims.import_reference()
-        theirs = ref.autoencoders.AudioAutoencoder(_FakeEnc(), _FakeDec(), latent_dim=3, downsampling_ratio=4,
-                                                   sample_rate=16000, io_channels=2, bottleneck=None)
-        assert torch.equal(enc_c, theirs.encode_audio(a.clone(), chunked=True, chunk_size=8, overlap=2, max_batch_size=3))
-        assert torch.equal(dec_c, theirs.decode_audio(z.clone(), chunked=True, chunk_size=8, overlap=2, max_batch_size=2))
-        assert torch.equal(rec_c, theirs.reconstruct_audio(a.clone(), chunked=True, chunk_size=8, overlap=2, max_batch_size=4))
+    assert torch.equal(enc_c, torch.from_numpy(g["enc"]))
+    assert torch.equal(dec_c, torch.from_numpy(g["dec"]))
+    assert torch.equal(rec_c, torch.from_numpy(g["rec"]))
 
 
 def test_vae_bottleneck_sampling_follows_the_torch_rng():
